@@ -23,6 +23,7 @@ there and in cpu_baseline).
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -32,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "raft-tf_b200"))
 
@@ -74,6 +76,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "20", "-i", str(self.idx)], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.kill)  # never leave the sampler running, also when the benchmark fails before stop()
             self.t = threading.Thread(target=lambda: [self.lines.append(l) for l in self.proc.stdout], daemon=True)
             self.t.start()
         except Exception:
@@ -125,7 +128,7 @@ def effective_cores():
 def cpu_sample(threads):
     """One step of the workload on the host CPU: the full 440x1024 pair through encoders, correlation pyramid, ALL 32
     iterations and the convex upsampling of the CPU oracle (torch fp32 restatement of the reference; nothing is
-    extrapolated).  Returns (seconds per pair, description)."""
+    extrapolated).  Returns (seconds per pair, description, [1,440,1024,2] flow)."""
     from oracle.raft_oracle import RAFTOracle, upsample_flow
     from raft_b200 import synth
     torch.set_num_threads(threads)
@@ -136,11 +139,20 @@ def cpu_sample(threads):
     st = m.prepare(torch.from_numpy(l), torch.from_numpy(r))
     t1 = time.perf_counter()
     net, mask, c1 = m.iterate(st)
-    upsample_flow(c1 - st["coords0"], mask)
+    flow = upsample_flow(c1 - st["coords0"], mask)
     t2 = time.perf_counter()
     desc = (f"1 frame pair {H_PAD}x{W_PAD}, all {ITERS} iterations measured (encoders + volume {t1 - t0:.2f}s, iterations + "
             f"upsampling {t2 - t1:.2f}s); torch-CPU fp32 oracle, {threads} threads")
-    return t2 - t0, desc
+    return t2 - t0, desc, flow
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each array as out_dir/<name>.npy (float32) so that two builds run with the same arguments
+    can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32, copy=False))
 
 
 def run_reference(args, rank, world):
@@ -155,8 +167,10 @@ def run_reference(args, rank, world):
     ts = []
     desc = ""
     for _ in range(args.steps):
-        t, desc = cpu_sample(threads)
+        t, desc, flow = cpu_sample(threads)
         ts.append(t)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"flow": flow})
     dt = sum(ts)
     v = args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "pairs/s", "n_gpus": args.gpus,
@@ -188,7 +202,7 @@ def other_configs(args, rank, world, dev, timed, dist):
     if world == 1:
         specs.insert(0, ("config3", False, 8, 540, 960, 32))
     out = {}
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
     for name, small, b, H, W, iters in specs:
         try:
             m = RAFT((H, W, 3), SimpleNamespace(small=small), iters=iters, batch=b, device=dev).load(synth.make_weights(small))
@@ -233,15 +247,26 @@ def other_configs(args, rank, world, dev, timed, dist):
     return out
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive_int, default=20, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch-per-gpu", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the other BASELINE configs (other_configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the flow of the last timed headline step to DIR/flow.npy "
+                         "(float32; DIR/flow_rank<r>.npy for ranks > 0; the leading samples of the batch that fit "
+                         "in 64 MiB over all ranks)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
@@ -292,8 +317,10 @@ def main():
             t = float(tt.item())
         return t
 
+    last = {}
+
     def step_resident():
-        model.forward(l_dev, r_dev)
+        last["flow"] = model.forward(l_dev, r_dev)  # a fresh tensor per call (RAFT.forward): what a caller receives
 
     def step_e2e():
         flow = model.forward(l_host, r_host)  # H2D of both frames inside
@@ -309,6 +336,7 @@ def main():
     launches_per_fwd = eng.launches_per_forward()
     m0 = clocks.mark()
     t_res = timed(step_resident, args.steps)
+    flow_last = last["flow"]  # output of the last timed step (the untimed steps below must not replace it)
     m1 = clocks.mark()
     clk = None
     if rank == 0:
@@ -430,11 +458,15 @@ def main():
     if not args.headline_only:
         others = other_configs(args, rank, world, dev, timed, dist)
 
+    if args.dump_outputs:
+        keep = max(1, (64 << 20) // world // (flow_last[0].numel() * 4))  # <= 64 MiB over all ranks: leading samples
+        dump_outputs(args.dump_outputs, {"flow" if rank == 0 else f"flow_rank{rank}": flow_last[:keep]})
+
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         threads = min(effective_cores(), 32)
         cpu_sample(threads)  # warm-up (page-in, oneDNN primitive caches)
-        tc, desc = cpu_sample(threads)
+        tc, desc, _ = cpu_sample(threads)
         cpu = {"value": 1.0 / tc, "unit": "pairs/s", "cores": threads, "kind": "port", "sample": desc}
 
     if rank == 0:
