@@ -8,12 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["capi.cu", "corr.cu", "conv_simt.cu", "conv_tc.cu", "conv_api.cu", "gemm_tc.cu", "update.cu", "upsample.cu",
            "encoder.cu", "frames.cu"]
-# Measured-slower kernel variants of round 1 (halo tiles, cta_group::2 pairs, weight multicast, the fused per-iteration
-# kernel; profiles/r01_notes.md).  They are NOT part of libraft_b200.so: `python build.py --experiments` builds a second
-# library, libraft_b200_exp.so (-DRB_EXPERIMENTS), that tools/ and tests/test_gpu_variants.py select with RAFT_B200_LIB.
-EXPERIMENT_SOURCES = ["experiments/conv_tc2.cu", "experiments/update_fused.cu", "experiments/conv_halo.cu"]
 LIB = os.path.join(HERE, "lib", "libraft_b200.so")
-LIB_EXP = os.path.join(HERE, "lib", "libraft_b200_exp.so")
 
 
 def needs_build() -> bool:
@@ -25,18 +20,14 @@ def needs_build() -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, experiments: bool = False) -> str:
-    lib = LIB_EXP if experiments else LIB
-    if not force and not experiments and not needs_build():
-        return lib
-    os.makedirs(os.path.dirname(lib), exist_ok=True)
+def build(force: bool = False, verbose: bool = False) -> str:
+    if not force and not needs_build():
+        return LIB
+    os.makedirs(os.path.dirname(LIB), exist_ok=True)
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    srcs = SOURCES + (EXPERIMENT_SOURCES if experiments else [])
-    objdir = os.path.join(HERE, "lib", "obj_exp" if experiments else "obj")
+    objdir = os.path.join(HERE, "lib", "obj")
     os.makedirs(objdir, exist_ok=True)
     flags = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
-    if experiments:
-        flags.append("-DRB_EXPERIMENTS")
     if verbose:
         flags += ["-Xptxas", "-v"]
     # one nvcc per translation unit, in parallel (the tcgen05 kernels dominate the build time); objects are rebuilt
@@ -45,18 +36,18 @@ def build(force: bool = False, verbose: bool = False, experiments: bool = False)
     hdrs.append(os.path.join(HERE, "..", "include", "raft_b200.h"))
     hdr_t = max(os.path.getmtime(h) for h in hdrs)
     procs, objs = [], []
-    for s in srcs:
+    for s in SOURCES:
         src = os.path.join(HERE, "csrc", s)
-        obj = os.path.join(objdir, os.path.basename(s)[:-3] + ".o")
+        obj = os.path.join(objdir, s[:-3] + ".o")
         objs.append(obj)
         if force or not os.path.exists(obj) or os.path.getmtime(obj) < max(os.path.getmtime(src), hdr_t):
             procs.append((s, subprocess.Popen([nvcc] + flags + ["-c", src, "-o", obj])))
     failed = [s for s, p in procs if p.wait() != 0]
     if failed:
         raise RuntimeError(f"nvcc failed for {failed}")
-    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "static", "-o", lib] + objs, check=True)
-    return lib
+    subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "static", "-o", LIB] + objs, check=True)
+    return LIB
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, experiments="--experiments" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

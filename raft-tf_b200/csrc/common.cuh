@@ -109,7 +109,6 @@ struct ConvParams {
   // (The iteration-invariant `inp` slice of the GRU inputs is convolved once per pair and skipped afterwards.)
   int ck_begin, ck_count, ck_skip_at, ck_skip;
   const float* addend;  // optional fp32 [pixel][cout] added to the accumulator before bias/activation
-  int pdl_early;
   const float* flow_tail;  // EPI_ACT, 16-channel epilogue: coords1; the last two channels are written as flow = coords1 - grid
   double* stat_part;  // EPI_F32 + tensor-core wide epilogue: per-(sample, strip, channel) sum / sum of squares of the
   int stat_strips;    // stored values, [B][strips][2][cout] (strip = 4 * tile-in-image + lane quarter); encoder.cu
@@ -118,7 +117,6 @@ struct ConvParams {
   int split_close;    // launcher: closing cluster barrier of the split-K pair (RAFT_B200_SPLITK_CLOSING_BARRIER, sanitizer runs)
   int split_cluster;  // ... set by the launcher: the halves run on the two CTAs of a cluster (one wave of pairs, batch 1)
   int cta_limit;  // > 0: at most this many persistent CTAs (a conv that runs beside another one on a forked stream)
-  int whatif;  // timing experiments only (fused kernel): 64 no global stores, 128 no global loads in the wide epilogue
   long long* dbg;       // optional phase timestamps (globaltimer ns), 8 slots per CTA; see tools/phase_times.py
   // packed weights [cout_pad][kh*kw][cin_pad] (K-major) as split planes + fp32 bias
   const __half* w_hi;
@@ -153,9 +151,6 @@ __host__ __device__ inline int conv_pad_y(const ConvParams& p) { return p.pad_ex
 __host__ __device__ inline int conv_in_w(const ConvParams& p) { return p.in_w > 0 ? p.in_w : p.w; }
 __host__ __device__ inline int conv_in_h(const ConvParams& p) { return p.in_h > 0 ? p.in_h : p.h; }
 __host__ __device__ inline int conv_rowpitch(const ConvParams& p) { return p.in_rowpitch > 0 ? p.in_rowpitch : p.in_stride * conv_in_w(p); }
-__host__ __device__ inline bool conv_default_view(const ConvParams& p) {
-  return p.in_w == 0 && p.in_h == 0 && p.in_rowpitch == 0 && p.in_cext == 0 && p.sx <= 1 && p.sy <= 1 && !p.pad_explicit;
-}
 
 // Gate non-linearities on the SFU: exp via ex2.approx (abs. error of the gate < 3e-7 for |x| < 16, i.e.
 // below the 2^-22 operand truncation of the split GEMM that feeds them), reciprocal via rcp.approx.
@@ -366,36 +361,20 @@ __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t&
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
-template <bool WI>
-__device__ __forceinline__ void store_split16(const ConvParams& p, __half* dhi, __half* dlo, size_t off, const float* y) {
+__device__ __forceinline__ void store_split16(__half* dhi, __half* dlo, size_t off, const float* y) {
   uint32_t h[8], l[8];
 #pragma unroll
   for (int i = 0; i < 8; ++i) split2(y[2 * i], y[2 * i + 1], h[i], l[i]);
-  if (!WI || !(p.whatif & 64)) {
-    st256_b32(dhi + off, h);
-    st256_b32(dlo + off, l);
-  } else if (h[0] == 0x12345678u) {  // timing experiment: keep the math alive
-    dhi[off] = __float2half(1.f);
-  }
+  st256_b32(dhi + off, h);
+  st256_b32(dlo + off, l);
 }
-template <bool WI>
-__device__ __forceinline__ void load16(const ConvParams& p, const float* src, float* d) {
-  if (!WI || !(p.whatif & 128)) {
-    ld256(src, d);
-    ld256(src + 8, d + 8);
-  } else {
-#pragma unroll
-    for (int i = 0; i < 16; ++i) d[i] = 0.5f;
-  }
+__device__ __forceinline__ void load16(const float* src, float* d) {
+  ld256(src, d);
+  ld256(src + 8, d + 8);
 }
-template <bool WI>
-__device__ __forceinline__ void store16(const ConvParams& p, float* dst, const float* v) {
-  if (!WI || !(p.whatif & 64)) {
-    st256(dst, v);
-    st256(dst + 8, v + 8);
-  } else if (v[0] == 12345.678f) {
-    dst[0] = 1.f;
-  }
+__device__ __forceinline__ void store16(float* dst, const float* v) {
+  st256(dst, v);
+  st256(dst + 8, v + 8);
 }
 // ---- TMEM as a prefetch buffer for epilogue operands ("stash") -------------------------------------------------------
 // At batch 1 a conv CTA owns ONE tile, so the second accumulator buffer in TMEM is never used by the MMA warp.  The 16
@@ -428,10 +407,8 @@ struct Stash {
   int cl;          // column of the current 16-channel chunk inside the tile
 };
 
-// WI: compile the RAFT_B200_WHATIF hooks in (fused kernel only; everything the default path runs stays lean)
 // `live` = this lane's pixel exists.  Without a stash the caller only calls live lanes; WITH a stash every lane of the warp
 // must come here (tcgen05.ld is .sync.aligned: warp-collective) and dead lanes skip the global accesses.
-template <bool WI = false>
 __device__ __forceinline__ void epilogue_wide16(const ConvParams& p, int pix, int c, float* y, const Stash st = Stash{0, 0, 0},
                                                 const bool live = true) {
   if (p.bias) {
@@ -444,14 +421,11 @@ __device__ __forceinline__ void epilogue_wide16(const ConvParams& p, int pix, in
   if (p.addend) {
     float t[16];
     const float* ad = p.addend + (size_t)pix * p.cout + c;
-    if (!WI && st.taddr) {
+    if (st.taddr) {
       tmem_ld16_sync(st.taddr + st.cl, t);
-    } else if (!WI || !(p.whatif & 128)) {
+    } else {
       ld256_nc(ad, t);
       ld256_nc(ad + 8, t + 8);
-    } else {
-#pragma unroll
-      for (int i = 0; i < 16; ++i) t[i] = 0.25f;
     }
 #pragma unroll
     for (int i = 0; i < 16; ++i) y[i] += t[i];
@@ -478,33 +452,33 @@ __device__ __forceinline__ void epilogue_wide16(const ConvParams& p, int pix, in
         y[14] = cc.x - (float)x;
         y[15] = cc.y - (float)yy;
       }
-      store_split16<WI>(p, p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + c, y);
-      if (p.d1_hi) store_split16<WI>(p, p.d1_hi, p.d1_lo, (size_t)pix * p.d1_stride + p.d1_choff + c, y);
+      store_split16(p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + c, y);
+      if (p.d1_hi) store_split16(p.d1_hi, p.d1_lo, (size_t)pix * p.d1_stride + p.d1_choff + c, y);
     } break;
     case EPI_ZR: {
       if (c < p.hidden) {
 #pragma unroll
         for (int i = 0; i < 16; ++i) y[i] = sigmoid_f(y[i]);
-        if (live) store16<WI>(p, p.f0 + (size_t)pix * p.hidden + c, y);
+        if (live) store16(p.f0 + (size_t)pix * p.hidden + c, y);
       } else {
         const int ch = c - p.hidden;
         float hprev[16];
-        if (!WI && st.taddr) tmem_ld16_sync(st.taddr + st.bn + st.cl, hprev);
-        else load16<WI>(p, p.f1 + (size_t)pix * p.hidden + ch, hprev);
+        if (st.taddr) tmem_ld16_sync(st.taddr + st.bn + st.cl, hprev);
+        else load16(p.f1 + (size_t)pix * p.hidden + ch, hprev);
 #pragma unroll
         for (int i = 0; i < 16; ++i) y[i] = sigmoid_f(y[i]) * hprev[i];
-        if (live) store_split16<WI>(p, p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + ch, y);
+        if (live) store_split16(p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + ch, y);
       }
     } break;
     case EPI_Q: {
       float z[16], hprev[16];
       float* hp = p.f1 + (size_t)pix * p.hidden + c;
-      if (!WI && st.taddr) {
+      if (st.taddr) {
         tmem_ld16_sync(st.taddr + st.bn + st.cl, z);
         tmem_ld16_sync(st.taddr + 2 * st.bn + st.cl, hprev);
       } else {
-        load16<WI>(p, p.f0 + (size_t)pix * p.hidden + c, z);
-        load16<WI>(p, hp, hprev);
+        load16(p.f0 + (size_t)pix * p.hidden + c, z);
+        load16(hp, hprev);
       }
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
@@ -512,8 +486,8 @@ __device__ __forceinline__ void epilogue_wide16(const ConvParams& p, int pix, in
         y[i] = (1.0f - z[i]) * hprev[i] + z[i] * q;  // model_utils.py:147,155,168
       }
       if (live) {
-        store16<WI>(p, hp, y);
-        store_split16<WI>(p, p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + c, y);
+        store16(hp, y);
+        store_split16(p.d0_hi, p.d0_lo, (size_t)pix * p.d0_stride + p.d0_choff + c, y);
       }
     } break;
     default: {  // EPI_F32
@@ -528,7 +502,7 @@ __device__ __forceinline__ void epilogue_wide16(const ConvParams& p, int pix, in
 #pragma unroll
         for (int i = 0; i < 16; ++i) y[i] = p.scale * y[i];
       }
-      store16<WI>(p, p.f0 + (size_t)pix * p.cout + c, y);
+      store16(p.f0 + (size_t)pix * p.cout + c, y);
     } break;
   }
 }

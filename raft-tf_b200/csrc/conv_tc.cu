@@ -52,12 +52,9 @@ struct TcCfg {
 };
 
 
-// PAIR = true: CTAs are launched as clusters of two that work on two pixel tiles of the SAME cout tile; CTA 0 fetches
-// B_hi, CTA 1 fetches B_lo, each with TMA multicast into both CTAs' shared memory, so every SM issues only half of
-// the weight-tile requests (the measured bound of the MMA loop is the ~38 B/clk a single SM can request from L2).
 // EXTRAS: phase timestamps (p.dbg) and fused instance-norm statistics (p.stat_part) -- a separate instantiation, so that
 // the kernel the update block runs stays below the 96-register cap of a 576-thread CTA without spills.
-template <int BLOCK_N, bool PAIR, bool EXTRAS>
+template <int BLOCK_N, bool EXTRAS>
 __global__ void __launch_bounds__(kTcThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
                const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
@@ -83,7 +80,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
   //  * p.split_cluster = 1 (one wave of CTA pairs, batch 1): clusters of two CTAs share one pixel tile, CTA r multiplies
   //    half r; CTA 1 hands its partial sums to CTA 0 through distributed shared memory, CTA 0 runs the epilogue on r0 + r1;
   //  * else one CTA runs both halves back to back into two TMEM accumulators and its epilogue adds them the same way.
-  const bool halves = !PAIR && BLOCK_N == 16 && p.split_k;
+  const bool halves = BLOCK_N == 16 && p.split_k;
   const bool splitk = halves && p.split_cluster;
   const int chunks = splitk ? conv_chunks(p) / 2 : conv_chunks(p);
   const int taps = p.kh * p.kw;
@@ -92,7 +89,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&tmA_hi); prefetch_tmap(&tmA_lo); prefetch_tmap(&tmB_hi); prefetch_tmap(&tmB_lo);
-    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], PAIR ? 2 : 1); }
+    for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full_bar[i], 1); mbar_init(&tmem_empty_bar[i], Cfg::kGroups * 4); }
     mbar_init(red_bar, 128);
     fence_barrier_init();
@@ -101,17 +98,15 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
   if (warp == 1) tmem_alloc(tmem_slot, Cfg::kTmemCols);
   tc_fence_before();
   __syncthreads();
-  if (PAIR || splitk) cluster_sync_all();  // the peer's barriers must be initialised before anything of ours can reach them
+  if (splitk) cluster_sync_all();  // the peer's barriers must be initialised before anything of ours can reach them
   tc_fence_after();
   // warp-wide OR of identical values: lands in a UNIFORM register, so that ptxas does not wrap every tcgen05.mma of the
   // single issuing lane in an elect / R2UR.BROADCAST "waterfall" loop (that was ~50 cycles per MMA, 8 MMAs per k-iteration)
   const uint32_t tmem_base = __reduce_or_sync(0xffffffffu, *tmem_slot);
-  const int rank = PAIR ? (int)cluster_ctarank() : 0;
   const int krank = splitk ? (int)cluster_ctarank() : 0;
-  const int first = (PAIR || splitk) ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;      // first work item of this CTA (pair)
-  const int stride = (PAIR || splitk) ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const int first = splitk ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;      // first work item of this CTA (pair)
+  const int stride = splitk ? (int)(gridDim.x >> 1) : (int)gridDim.x;
   if (dbg && threadIdx.x == 0) dbg[1] = gtime_ns();
-  if (p.pdl_early) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   // Programmatic dependent launch: this kernel may have been started while its predecessor is still running.  Everything
   // up to here (barriers, TMEM, tensor-map prefetch) and the WEIGHT tiles of the first ring stages are independent of
   // it; `griddepcontrol.wait` (no-op without the launch attribute) is executed by the producer before its first
@@ -124,16 +119,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
       uint32_t phase = 0;  // the k-iteration -> (chunk, kx, ky) mapping is advanced incrementally.
       bool waited = false;
       for (int tile = first; tile < g.total_tiles; tile += stride) {
-        const int mq = tile / g.n_tiles, nt = tile - mq * g.n_tiles;
-        const int mt = PAIR ? 2 * mq + rank : mq;  // a trailing odd tile gets a dummy partner: b >= B, TMA zero-fills
+        const int mt = tile / g.n_tiles, nt = tile - mt * g.n_tiles;
         const int b = mt / tiles_per_img, trem = mt - b * tiles_per_img;
         const int ty = trem / g.tiles_x, tx = trem - ty * g.tiles_x;
         const int y0 = ty << g.bh_log2, x0 = tx << g.bw_log2, n0 = nt * BLOCK_N;
         const int xs = x0 * csx - pw, ys = y0 * csy - ph;  // input coordinates of tap (0, 0) of the tile's first pixel
         const int wb = p.w_per_batch ? min(b, p.B - 1) : 0;
-        // K order: channel chunk outermost, then kx, then ky -- the same order as conv_halo.cu, so that the two
-        // kernels (chosen by tile count, i.e. by batch size) accumulate identically and a batched run equals the
-        // per-sample runs bit for bit.
+        // K order: channel chunk outermost, then kx, then ky.  The order is fixed, whatever the tile geometry or the
+        // number of tiles per CTA, so a batched run equals the per-sample runs bit for bit.
         struct KIter {
           int cki, kx, ky, ck;
         };
@@ -152,13 +145,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         auto load_b = [&](const KIter& k, int slot) {
           uint8_t* st = smem + slot * Cfg::kStageBytes;
           const int kcol = (k.ky * p.kw + k.kx) * p.cin_pad + k.ck * kChunkK;
-          if (PAIR) {  // half of the weight tile each, delivered to both CTAs
-            if (rank == 0) tma_load_3d_mc(&tmB_hi, &full_bar[slot], st + 2 * kATileBytes, kcol, n0, wb, (uint16_t)3);
-            else tma_load_3d_mc(&tmB_lo, &full_bar[slot], st + 2 * kATileBytes + Cfg::kBTileBytes, kcol, n0, wb, (uint16_t)3);
-          } else {
-            tma_load_3d(&tmB_hi, &full_bar[slot], st + 2 * kATileBytes, kcol, n0, wb);
-            tma_load_3d(&tmB_lo, &full_bar[slot], st + 2 * kATileBytes + Cfg::kBTileBytes, kcol, n0, wb);
-          }
+          tma_load_3d(&tmB_hi, &full_bar[slot], st + 2 * kATileBytes, kcol, n0, wb);
+          tma_load_3d(&tmB_lo, &full_bar[slot], st + 2 * kATileBytes + Cfg::kBTileBytes, kcol, n0, wb);
         };
         KIter k = {krank * chunks, 0, 0, conv_chunk(p, krank * chunks)};
         int it0 = 0;
@@ -166,7 +154,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
           // first tile of the kernel: weight tiles of the first ring stages, then wait for the predecessor kernel, then
           // the activation tiles of the same stages (the ring is empty here: slots 0.., phase 0)
           // (not when the B operand is itself an activation produced by an earlier kernel: corr build, w_per_batch)
-          const int pre = (PAIR || p.w_per_batch) ? 0 : (kiters < STAGES ? kiters : STAGES);
+          const int pre = p.w_per_batch ? 0 : (kiters < STAGES ? kiters : STAGES);
           KIter kb = k;
           for (int it = 0; it < pre; ++it) {
             mbar_arrive_expect_tx(&full_bar[it], Cfg::kStageBytes);
@@ -223,8 +211,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
             umma_f16(acc, a_hi + koff, b_all + koff, idesc_2n, (BLOCK_N == 16 ? ((it != 0 && it != it_half) || k != 0) : (it | k) != 0));
             umma_f16(acc + BLOCK_N, a_lo + koff, b_all + koff, idesc_n, 1u);
           }
-          if (PAIR) umma_commit_mc(&empty_bar[s], (uint16_t)3);  // both producers write into this stage of both CTAs
-          else umma_commit(&empty_bar[s]);                      // frees the smem stage when these MMAs retire
+          umma_commit(&empty_bar[s]);  // frees the smem stage when these MMAs retire
           if (++s == STAGES) { s = 0; phase ^= 1; }
         }
         umma_commit(&tmem_full_bar[ab]);
@@ -283,8 +270,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         }
       }
       for (int tile = first; tile < g.total_tiles; tile += stride, ++li) {
-        const int mq = tile / g.n_tiles, nt = tile - mq * g.n_tiles;
-        const int mt = PAIR ? 2 * mq + rank : mq;
+        const int mt = tile / g.n_tiles, nt = tile - mt * g.n_tiles;
         const int b = mt / tiles_per_img, trem = mt - b * tiles_per_img;
         const int ty = trem / g.tiles_x, tx = trem - ty * g.tiles_x;
         const int y0 = ty << g.bh_log2, x0 = tx << g.bw_log2, n0 = nt * BLOCK_N;
@@ -311,7 +297,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
 #pragma unroll
           for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(d0[i]) + __uint_as_float(d1[i]) * kLoInv;
           bool store = valid;
-          if constexpr (BLOCK_N == 16 && !PAIR) {
+          if constexpr (BLOCK_N == 16) {
             if (halves && !splitk) {  // second accumulator of the same CTA
               tmem_ld16(trow + Cfg::kAccCols + c, d0);
               tmem_ld16(trow + Cfg::kAccCols + BLOCK_N + c, d1);
@@ -367,7 +353,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
   if (dbg && warp == 2 && lane == 0) dbg[6] = gtime_ns();
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();  // the peer may still multicast into this CTA's smem / arrive on its barriers
   // Split-K: CTA 0 cannot exit before CTA 1's partial sums have landed in its shared memory -- it waited for them
   // (mbarrier, release.cluster / acquire.cluster) -- so no closing cluster barrier is needed.  compute-sanitizer's racecheck
   // cannot see that ("block that might have already exited"); p.split_close adds the barrier it wants (0 hazards with it,
@@ -412,13 +397,9 @@ int make_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t* dims
   const CUtensorMapDataType dt = kind == TMAP_F16_SW128 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   const CUtensorMapSwizzle sw = kind == TMAP_F16_SW128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
   // L2 promotion: 256-byte requests suit the dense 128-byte operand rows of the GEMM tiles; the lookup's 64-byte patch
-  // rows are a gather (r01: 1.86x the algorithmic DRAM bytes) -> none.  RAFT_B200_LOOKUP_L2PROMO = 0/64/128/256: A/B knob.
-  CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-  if (kind == TMAP_F32_SW64_GATHER) {
-    static const int env = getenv("RAFT_B200_LOOKUP_L2PROMO") ? atoi(getenv("RAFT_B200_LOOKUP_L2PROMO")) : 0;
-    promo = env == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : env == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B
-            : env == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : CU_TENSOR_MAP_L2_PROMOTION_NONE;
-  }
+  // rows are a gather (r01: 1.86x the algorithmic DRAM bytes) -> none.
+  const CUtensorMapL2promotion promo =
+      kind == TMAP_F32_SW64_GATHER ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
   CUresult r = fn(out, dt, (cuuint32_t)rank, const_cast<void*>(base), gdim, gstr, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                   promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   RB_REQUIRE(r == CUDA_SUCCESS, RB_ERR_CUDA,
@@ -520,30 +501,30 @@ static int choose_block_n(int cout, long m_tiles, int ctas = 148) {  // ctas: pe
   return best;
 }
 
-template <int BLOCK_N, bool PAIR>
+template <int BLOCK_N>
 static int launch_cfg(const ConvParams& p_in, TileGeom g, const CUtensorMap* maps, cudaStream_t s) {
   using Cfg = TcCfg<BLOCK_N>;
   static PerDeviceOnce attr_set;
   int dev = 0, rc_dev;
   if ((rc_dev = current_device(&dev))) return rc_dev;
   if (!attr_set.test(dev)) {
-    RB_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, PAIR, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
-    RB_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, PAIR, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+    RB_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+    RB_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     attr_set.set(dev);
   }
   const int num_sms = device_sm_count(dev);
   ConvParams p = p_in;
   g.n_tiles = (p.cout + BLOCK_N - 1) / BLOCK_N;
   g.m_tiles = p.B * g.tiles_x * g.tiles_y;
-  g.total_tiles = (PAIR ? (g.m_tiles + 1) / 2 : g.m_tiles) * g.n_tiles;
+  g.total_tiles = g.m_tiles * g.n_tiles;
   // split-K: only when every pixel tile gets its own CTA pair in one wave (batch 1), else the plain persistent grid
-  if (p.split_k && !(BLOCK_N == 16 && !PAIR && p.cout <= 2 && p.epi == EPI_DELTA && !p.w_per_batch && conv_chunks(p) % 2 == 0))
+  if (p.split_k && !(BLOCK_N == 16 && p.cout <= 2 && p.epi == EPI_DELTA && !p.w_per_batch && conv_chunks(p) % 2 == 0))
     p.split_k = 0;
   static const bool no_cluster = getenv("RAFT_B200_NO_SPLITK_CLUSTER") != nullptr;  // test knob: same sums on one CTA
   static const bool close_barrier = getenv("RAFT_B200_SPLITK_CLOSING_BARRIER") != nullptr;  // for compute-sanitizer runs
   p.split_close = close_barrier ? 1 : 0;
   p.split_cluster = (p.split_k && 2 * g.total_tiles <= num_sms && p.cta_limit <= 0 && !no_cluster) ? 1 : 0;
-  const bool cluster2 = PAIR || p.split_cluster;
+  const bool cluster2 = p.split_cluster;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   int units = cluster2 ? num_sms / 2 : num_sms;  // persistent: at most one CTA (pair) per SM (pair)
@@ -564,76 +545,21 @@ static int launch_cfg(const ConvParams& p_in, TileGeom g, const CUtensorMap* map
   // weight tiles overlap the tail of this one.  Same-box A/B after the issue-loop fixes: 190 -> 175 us per update step.
   static const int pdl = getenv("RAFT_B200_NO_PDL") ? 0 : 1;
   cfg.numAttrs = 1 + pdl;
-  int stages = Cfg::kStages;
-  static const int env_stages = getenv("RAFT_B200_TC_STAGES") ? atoi(getenv("RAFT_B200_TC_STAGES")) : 0;  // tuning knob
-  if (env_stages > 0 && env_stages < stages) stages = env_stages;
+  const int stages = Cfg::kStages;
   if (p.dbg || p.stat_part)
-    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BLOCK_N, PAIR, true>, maps[0], maps[1], maps[2], maps[3], p, g, stages));
+    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BLOCK_N, true>, maps[0], maps[1], maps[2], maps[3], p, g, stages));
   else
-    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BLOCK_N, PAIR, false>, maps[0], maps[1], maps[2], maps[3], p, g, stages));
+    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BLOCK_N, false>, maps[0], maps[1], maps[2], maps[3], p, g, stages));
   RB_CHECK_LAUNCH("conv_tc_kernel");
   return RB_OK;
 }
 
-#ifdef RB_EXPERIMENTS  // measured-slower variants (csrc/experiments/, profiles/r01_notes.md): only in libraft_b200_exp.so
-int launch_conv_halo(const ConvParams& p, cudaStream_t s, bool* handled);
-int launch_conv_tc2(const ConvParams& p, cudaStream_t s, int bn, int bw_log2, int bh_log2, int tiles_x, int tiles_y, bool* handled);
-#endif
-
-#ifdef RB_EXPERIMENTS
-// Geometry, tile width and tensor maps of one conv for the fused update-step kernel (experiments/update_fused.cu).
-int conv_tc_prepare(const ConvParams& p, FusedJob* job) {
-  RB_REQUIRE(p.cin_pad % kChunkK == 0 && p.in_stride % 8 == 0 && p.in_choff % 8 == 0, RB_ERR_BAD_SHAPE,
-             "conv_tc: channel padding (cin_pad=%d stride=%d off=%d)", p.cin_pad, p.in_stride, p.in_choff);
-  TileGeom g = choose_geom(p.h, p.w);
-  g.m_tiles = p.B * g.tiles_x * g.tiles_y;
-  const int bn = choose_block_n(p.cout, g.m_tiles, p.cta_limit > 0 && p.cta_limit < 148 ? p.cta_limit : 148);
-  g.n_tiles = (p.cout + bn - 1) / bn;
-  g.total_tiles = g.m_tiles * g.n_tiles;
-  job->p = p;
-  job->g = g;
-  job->block_n = bn;
-  {
-    uint64_t dims[4] = {(uint64_t)p.in_stride, (uint64_t)p.w, (uint64_t)p.h, (uint64_t)p.B};
-    uint64_t str[3] = {(uint64_t)p.in_stride * 2, (uint64_t)p.in_stride * 2 * p.w, (uint64_t)p.in_stride * 2 * p.w * p.h};
-    uint32_t box[4] = {(uint32_t)kChunkK, 1u << g.bw_log2, 1u << g.bh_log2, 1};
-    int rc;
-    if ((rc = cached_tmap(&job->m[0], p.in_hi, 4, dims, str, box))) return rc;
-    if ((rc = cached_tmap(&job->m[1], p.in_lo, 4, dims, str, box))) return rc;
-  }
-  {
-    const uint64_t ktot = (uint64_t)p.kh * p.kw * p.cin_pad;
-    uint64_t dims[3] = {ktot, (uint64_t)p.cout_pad, (uint64_t)(p.w_per_batch ? p.B : 1)};
-    uint64_t str[2] = {ktot * 2, ktot * 2 * p.cout_pad};
-    uint32_t box[3] = {(uint32_t)kChunkK, (uint32_t)bn, 1};
-    int rc;
-    if ((rc = cached_tmap(&job->m[2], p.w_hi, 3, dims, str, box))) return rc;
-    if ((rc = cached_tmap(&job->m[3], p.w_lo, 3, dims, str, box))) return rc;
-  }
-  return RB_OK;
-}
-#endif
-
 int launch_conv_tc(const ConvParams& p, cudaStream_t s) {
-#ifdef RB_EXPERIMENTS
-  if (p.kh * p.kw > 1 && !p.stat_part && conv_default_view(p)) {  // RAFT_B200_HALO=1: halo-tile kernel (each input pixel is fetched once per tap ROW)
-    bool handled = false;
-    int rc = launch_conv_halo(p, s, &handled);
-    if (rc || handled) return rc;
-  }
-#endif
   RB_REQUIRE(p.cin_pad % kChunkK == 0 && p.in_stride % 8 == 0 && p.in_choff % 8 == 0, RB_ERR_BAD_SHAPE,
              "conv_tc: channel padding (cin_pad=%d stride=%d off=%d)", p.cin_pad, p.in_stride, p.in_choff);
   const TileGeom g = choose_geom(p.h, p.w);
   const long m_tiles = (long)p.B * g.tiles_x * g.tiles_y;
   const int bn = choose_block_n(p.cout, m_tiles, p.cta_limit > 0 && p.cta_limit < 148 ? p.cta_limit : 148);
-#ifdef RB_EXPERIMENTS
-  if (!p.stat_part && conv_default_view(p)) {
-    bool handled = false;  // experimental cta_group::2 path (RAFT_B200_CTA2=1)
-    int rc = launch_conv_tc2(p, s, bn, g.bw_log2, g.bh_log2, g.tiles_x, g.tiles_y, &handled);
-    if (rc || handled) return rc;
-  }
-#endif
   CUtensorMap maps[4];
   {
     // the input view (common.cuh): strided convs traverse it with TMA element strides -- a box of bw*sx x bh*sy input
@@ -659,24 +585,12 @@ int launch_conv_tc(const ConvParams& p, cudaStream_t s) {
     if ((rc = cached_tmap(&maps[2], p.w_hi, 3, dims, str, box))) return rc;
     if ((rc = cached_tmap(&maps[3], p.w_lo, 3, dims, str, box))) return rc;
   }
-#ifdef RB_EXPERIMENTS
-  static const bool pair = getenv("RAFT_B200_PAIR") != nullptr;  // experiment: cluster-of-2 weight multicast
-  if (pair && m_tiles >= 2 && conv_default_view(p)) {
-    switch (bn) {
-      case 16: return launch_cfg<16, true>(p, g, maps, s);
-      case 32: return launch_cfg<32, true>(p, g, maps, s);
-      case 64: return launch_cfg<64, true>(p, g, maps, s);
-      case 96: return launch_cfg<96, true>(p, g, maps, s);
-      default: return launch_cfg<128, true>(p, g, maps, s);
-    }
-  }
-#endif
   switch (bn) {
-    case 16: return launch_cfg<16, false>(p, g, maps, s);
-    case 32: return launch_cfg<32, false>(p, g, maps, s);
-    case 64: return launch_cfg<64, false>(p, g, maps, s);
-    case 96: return launch_cfg<96, false>(p, g, maps, s);
-    default: return launch_cfg<128, false>(p, g, maps, s);
+    case 16: return launch_cfg<16>(p, g, maps, s);
+    case 32: return launch_cfg<32>(p, g, maps, s);
+    case 64: return launch_cfg<64>(p, g, maps, s);
+    case 96: return launch_cfg<96>(p, g, maps, s);
+    default: return launch_cfg<128>(p, g, maps, s);
   }
 }
 

@@ -719,9 +719,6 @@ int launch_lookup(const float* pyramid, const float* coords, float* out_f32, __h
       uint32_t box[3] = {16u, (uint32_t)(2 * radius + 2), 1};
       if (cached_tmap(&maps.m[l], pv.base[l], 3, dims, str, box, tc::TMAP_F32_SW64_GATHER) != RB_OK) pv.tma_ok[l] = 0;  // plain loads
     }
-    static const bool no_tma = getenv("RAFT_B200_LOOKUP_NOTMA") != nullptr;  // diagnostic: stage every level with plain loads
-    if (no_tma)
-      for (int l = 0; l < RB_NUM_LEVELS; ++l) pv.tma_ok[l] = 0;
     if (radius == 4)
       return split ? launch_lookup_v5<4, true>(pv, maps, c2, nullptr, out_hi, out_lo, out_stride, npix, s)
                    : launch_lookup_v5<4, false>(pv, maps, c2, out_f32, nullptr, nullptr, out_stride, npix, s);

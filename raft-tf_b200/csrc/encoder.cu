@@ -106,11 +106,9 @@ static void enc_packed_layout(int small, int out_dim, std::vector<EncPacked>& P,
 // Stem input: the 2x-1 image (RAFT.py:53-59) as a zero-padded space-to-depth tensor.  Padded image row r' = r + pt
 // (TF SAME: pt = total/2 rows of zeros before), cell (Y, X) holds rows 2Y, 2Y+1 and columns 2X, 2X+1: channel
 // (dy*2 + dx)*3 + c of 16 (12..15 = 0).  Output pixel (oy, ox) of the 7x7 stride-2 conv reads cells (oy..oy+3, ox..ox+3).
-// One thread per cell; WINDOWS = false: cells once, [B][Hp][Wp][16] (the conv's view overlaps them);
-// WINDOWS = true: every view pixel materialised, [B][Hp][Wo][4 cells x 16] (RAFT_B200_STEM_WINDOWS=1).
-template <bool WINDOWS>
+// One thread per cell, each cell written once, [B][Hp][Wp][16] (the conv's view overlaps them).
 __global__ void enc_stem_s2d_kernel(const float* __restrict__ img, __half* __restrict__ out_hi, __half* __restrict__ out_lo, int B,
-                                    int H, int W, int pt, int pl, int Hp, int Wp, int Wo) {
+                                    int H, int W, int pt, int pl, int Hp, int Wp) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)B * Hp * Wp) return;
   const int X = i % Wp, Y = (i / Wp) % Hp, b = i / ((size_t)Wp * Hp);
@@ -133,20 +131,9 @@ __global__ void enc_stem_s2d_kernel(const float* __restrict__ img, __half* __res
     }
   const uint4* h4 = reinterpret_cast<const uint4*>(hi);
   const uint4* l4 = reinterpret_cast<const uint4*>(lo);
-  if (!WINDOWS) {
-    const size_t o = (((size_t)b * Hp + Y) * Wp + X) * 16;
-    reinterpret_cast<uint4*>(out_hi + o)[0] = h4[0]; reinterpret_cast<uint4*>(out_hi + o)[1] = h4[1];
-    reinterpret_cast<uint4*>(out_lo + o)[0] = l4[0]; reinterpret_cast<uint4*>(out_lo + o)[1] = l4[1];
-  } else {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {  // cell X is cell j of the window that starts at X - j
-      const int xw = X - j;
-      if (xw < 0 || xw >= Wo) continue;
-      const size_t o = (((size_t)b * Hp + Y) * Wo + xw) * 64 + j * 16;
-      reinterpret_cast<uint4*>(out_hi + o)[0] = h4[0]; reinterpret_cast<uint4*>(out_hi + o)[1] = h4[1];
-      reinterpret_cast<uint4*>(out_lo + o)[0] = l4[0]; reinterpret_cast<uint4*>(out_lo + o)[1] = l4[1];
-    }
-  }
+  const size_t o = (((size_t)b * Hp + Y) * Wp + X) * 16;
+  reinterpret_cast<uint4*>(out_hi + o)[0] = h4[0]; reinterpret_cast<uint4*>(out_hi + o)[1] = h4[1];
+  reinterpret_cast<uint4*>(out_lo + o)[0] = l4[0]; reinterpret_cast<uint4*>(out_lo + o)[1] = l4[1];
 }
 
 // instance-norm statistics, stage 1: per (sample, pixel strip) partial sum / sum of squares per channel
@@ -247,8 +234,8 @@ static EncWs enc_ws_layout(int small, int B, int H, int W, void* base) {
     w.act[i].hi = reinterpret_cast<__half*>(b + off); off += act_plane;
     w.act[i].lo = reinterpret_cast<__half*>(b + off); off += act_plane;
   }
-  // stem input cells: (Ho+3) x (Wo+3) x 16, or (Ho+3) x Wo x 64 with materialised windows
-  const size_t col_plane = al((size_t)B * ((H + 1) / 2 + 3) * ((W + 1) / 2 + 3) * 64 * sizeof(__half));
+  // stem input cells: (Ho+3) x (Wo+3) x 16; the overlapping view reads up to cell Wo+2 of a row
+  const size_t col_plane = al((size_t)B * ((H + 1) / 2 + 3) * ((W + 1) / 2 + 3) * 16 * sizeof(__half));
   w.col.hi = reinterpret_cast<__half*>(b + off); off += col_plane;
   w.col.lo = reinterpret_cast<__half*>(b + off); off += col_plane;
   w.f32 = reinterpret_cast<float*>(b + off); off += al(px2 * (size_t)(small ? 64 : 128) * sizeof(float));
@@ -291,19 +278,15 @@ static int enc_conv(const EncRun& R, int i, const float* img, SplitPtr in, int i
     int pt, pl;
     same_pad(h, c.k, c.stride, &pt, &oh);
     same_pad(w, c.k, c.stride, &pl, &ow);
-    static const bool windows = getenv("RAFT_B200_STEM_WINDOWS") != nullptr;  // A/B knob: materialised windows
     const int Hp = oh + 3, Wp = ow + 3;
     const size_t cells = (size_t)R.B * Hp * Wp;
-    if (windows)
-      enc_stem_s2d_kernel<true><<<(unsigned)((cells + 255) / 256), 256, 0, R.s>>>(img, R.ws.col.hi, R.ws.col.lo, R.B, h, w, pt, pl, Hp, Wp, ow);
-    else
-      enc_stem_s2d_kernel<false><<<(unsigned)((cells + 255) / 256), 256, 0, R.s>>>(img, R.ws.col.hi, R.ws.col.lo, R.B, h, w, pt, pl, Hp, Wp, ow);
+    enc_stem_s2d_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, R.s>>>(img, R.ws.col.hi, R.ws.col.lo, R.B, h, w, pt, pl, Hp, Wp);
     RB_CHECK_LAUNCH("enc_stem_s2d_kernel");
     p.in_hi = R.ws.col.hi; p.in_lo = R.ws.col.lo;
-    p.in_stride = windows ? 64 : 16;
+    p.in_stride = 16;
     p.in_cext = 64;
     p.in_w = ow; p.in_h = Hp;
-    p.in_rowpitch = windows ? ow * 64 : Wp * 16;
+    p.in_rowpitch = Wp * 16;
     p.pad_explicit = 1; p.pad_x = 0; p.pad_y = 0;
   } else if (c.stride != 1) {  // strided view of the activation, TF SAME offsets
     int pt, pl;

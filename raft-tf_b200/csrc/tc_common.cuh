@@ -98,15 +98,6 @@ __device__ __forceinline__ void tma_load_3d(const CUtensorMap* m, uint64_t* bar,
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
-
-// multicast variant: the box lands at the same smem offset (and signals the same barrier offset) in every CTA of `mask`
-__device__ __forceinline__ void tma_load_3d_mc(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1, int c2,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -161,12 +152,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
 }
-// commit that arrives on the barrier at the same offset in every CTA of `mask` (cluster multicast)
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask)
-               : "memory");
-}
 // 32 lanes x 16 consecutive 32-bit columns: thread t of the warp gets row (lane base + t).
 // The load is asynchronous: registers are valid only after tmem_ld_wait(), which names them as
 // in/out operands so the compiler cannot hoist uses above the wait.
@@ -200,33 +185,8 @@ struct TileGeom {
   int tiles_x, tiles_y;  // per image
   int n_tiles;           // cout tiles
   int m_tiles;           // B * tiles_x * tiles_y pixel tiles
-  int total_tiles;       // work items: m_tiles * n_tiles, or ceil(m_tiles/2) * n_tiles PAIRS in cluster mode
+  int total_tiles;       // work items: m_tiles * n_tiles
 };
-
-#ifdef RB_EXPERIMENTS
-// One conv of the fused update-step kernel (experiments/update_fused.cu)
-struct FusedJob {
-  CUtensorMap m[4];  // A_hi, A_lo, B_hi, B_lo
-  ConvParams p;
-  TileGeom g;
-  int block_n;
-  int wait_prev;   // 1: every earlier job of the list must be complete (grid barrier) before this job's loads
-  int cta_offset;  // tile t runs on CTA (t + cta_offset) % gridDim.x: independent jobs spread over different SMs
-  int pad_;
-};
-int conv_tc_prepare(const ConvParams& p, FusedJob* job);
-constexpr int kMaxFusedJobs = 12;
-struct FusedJobs {
-  FusedJob job[kMaxFusedJobs];
-  int n;
-  unsigned int* counters;  // [kMaxFusedJobs], zeroed before every launch
-  int stages;              // smem ring depth (<= 3)
-  long long* dbg;          // tools/fused_times.py: 8 globaltimer stamps per (job, CTA), 4096 CTAs per job
-  int whatif;              // timing experiments only (RAFT_B200_WHATIF bitmask, results are WRONG): 1 no A_lo*B_hi MMA,
-                           // 2 no A_lo load, 4 no B loads, 8 no A_hi load, 16 no MMAs at all, 32 no epilogue stores
-};
-int launch_fused_jobs(const FusedJobs& jobs, cudaStream_t s);
-#endif
 
 // per-thread cache of encoded tensor maps (conv_tc.cu)
 int cached_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides,
@@ -234,7 +194,7 @@ int cached_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t* di
 
 }  // namespace rb
 
-// ---- cta_group::2 (2-CTA tcgen05) building blocks ---------------------------------------------------------
+// ---- cluster building blocks (split-K pair of conv_tc.cu) -------------------------------------------------
 namespace rb {
 namespace tc {
 // shared::cluster address of the same shared-memory offset in CTA `rank` of the cluster
@@ -271,45 +231,6 @@ __device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity
 }
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA loads whose completion bytes are credited to a barrier that may live in the peer CTA of the pair
-__device__ __forceinline__ void tma_load_4d_2sm(const CUtensorMap* m, uint32_t bar_cluster_addr, void* dst, int c0, int c1,
-                                                int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_2sm(const CUtensorMap* m, uint32_t bar_cluster_addr, void* dst, int c0, int c1,
-                                                int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t* slot, uint32_t ncols) {  // same warp id in both CTAs
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t addr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(ncols) : "memory");
-}
-// M = 256 (128 rows per CTA), fp16 x fp16 -> fp32, both operands K-major
-__host__ __device__ constexpr uint32_t umma_idesc_f16_m256(int n) {
-  return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-}
-__device__ __forceinline__ void umma_f16_2sm(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2sm_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask)
-               : "memory");
 }
 }  // namespace tc
 }  // namespace rb

@@ -129,7 +129,6 @@ struct Workspace {
   float* H;
   float* Z;
   float* pre[4];  // things: bias + conv over the `inp` channels of zr1, q1, zr2, q2 (iteration-invariant)
-  unsigned int* counters;  // grid-barrier counters of the fused update-step kernel (update_fused.cu)
   size_t total;
 };
 
@@ -168,8 +167,6 @@ static Workspace workspace_layout(const Variant& v, size_t npix, void* base) {
       off += align_up(npix * (size_t)((i & 1) ? v.hidden : 2 * v.hidden) * sizeof(float), 1024);
     }
   }
-  W.counters = reinterpret_cast<unsigned int*>(b + off);
-  off += 1024;
   W.total = off;
   return W;
 }
@@ -237,9 +234,8 @@ __global__ void copy_f32_kernel(const float* __restrict__ src, float* __restrict
 }
 
 // encoder/convf1: 7x7 conv over the 2-channel flow + ReLU (model_utils.py:114,124), CUDA-core form: the cross-check back end
-// (RB_MATH_SIMT) and RAFT_B200_CONVF1_SIMT=1; the default is the tensor-core form (flow_prep_kernel below + conv_tc)
-// (K = 98 is no tensor-core shape).  flow = coords1 - coords_grid (RAFT.py:95) is formed while
-// staging; SAME padding zero-pads the FLOW.  One thread per output channel, SEG-pixel row segment
+// (RB_MATH_SIMT), and grids narrower than the 8-pixel window of the tensor-core form (flow_prep_kernel below + conv_tc).
+// flow = coords1 - coords_grid (RAFT.py:95) is formed while staging; SAME padding zero-pads the FLOW.  One thread per output channel, SEG-pixel row segment
 // per block (SEG = 16 at batch 1: 440 blocks instead of 220 -- the kernel is latency-bound, and with the convf2 that
 // follows it on the forked stream it must not finish later than lookup -> convc1 -> convc2 on the main stream); the flow itself is also written into the [.., flow] slot of HX/QX (concat_out, :119).
 template <int COUT, int SEG>
@@ -360,175 +356,11 @@ static void hoist_inp(const Variant& v, const Workspace& W, int idx, ConvParams&
   p.bias = nullptr;  // folded into the addend
 }
 
-// flow_head/conv2 (3x3, fh -> 2 channels, model_utils.py:134) + coords1 += delta (RAFT.py:102) on CUDA cores.
-// As an implicit GEMM this conv uses 2 of the 16 columns of the narrowest MMA tile and still streams a 32 KB
-// activation tile per (tap, 64-channel chunk) through every CTA (profiles/r01_notes.md: 12 us MMA phase on 55 SMs);
-// here the split planes are joined to fp32 once per 8x8-pixel halo tile in shared memory and 112 blocks (batch 1) do
-// 2 x 9 x CIN FMAs per pixel.  256 threads = 64 pixels x 4 channel quarters of every 64-channel chunk; fixed
-// summation order (bit-reproducible, batched == per-sample).  The weights are staged before griddepcontrol.wait.
-template <int CIN>
-__global__ void __launch_bounds__(256) flow_head2_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_lo,
-                                                         int in_stride, const __half* __restrict__ w_hi,
-                                                         const __half* __restrict__ w_lo, const float* __restrict__ bias,
-                                                         float* coords1, float* delta_out, int h, int w, int trigger) {
-  constexpr int kPitch = 68;  // floats per halo pixel (64 + 4: conflict-free 128-bit reads across pixels)
-  __shared__ __align__(16) float2 wsm[9 * CIN];
-  __shared__ __align__(16) float act[100 * kPitch];
-  __shared__ float2 red[4][64];
-  const int tid = threadIdx.x, px = tid & 63, q = tid >> 6;
-  const int b = blockIdx.z, y0 = blockIdx.y * 8, x0 = blockIdx.x * 8;
-  for (int i = tid * 8; i < 9 * CIN; i += 256 * 8) {  // packed [cout_pad][9][CIN] split planes -> fp32 (w[.., 0], w[.., 1])
-    const uint4 h0 = *reinterpret_cast<const uint4*>(w_hi + i), l0 = *reinterpret_cast<const uint4*>(w_lo + i);
-    const uint4 h1 = *reinterpret_cast<const uint4*>(w_hi + 9 * CIN + i), l1 = *reinterpret_cast<const uint4*>(w_lo + 9 * CIN + i);
-    const __half* a0 = reinterpret_cast<const __half*>(&h0);
-    const __half* b0 = reinterpret_cast<const __half*>(&l0);
-    const __half* a1 = reinterpret_cast<const __half*>(&h1);
-    const __half* b1 = reinterpret_cast<const __half*>(&l1);
-#pragma unroll
-    for (int k = 0; k < 8; ++k) wsm[i + k] = make_float2(join_f32(a0[k], b0[k]), join_f32(a1[k], b1[k]));
-  }
-  if (trigger == 0) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  const int ly = px >> 3, lx = px & 7;
-  float acc0 = 0.f, acc1 = 0.f;
-  // halo staging: 100 pixels x 8 vectors of 8 channels = 800 vectors, up to 4 per thread; the vectors of chunk c+1 are
-  // requested before the FMAs of chunk c (the kernel has 8 warps per SM: un-overlapped L2 latency would dominate it)
-  uint4 vh[4], vl[4];
-  size_t voff[4];
-  bool vin[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int v = tid + k * 256;
-    const int hp = v >> 3, c8 = (v & 7) * 8;
-    const int hy = hp / 10, hx = hp - hy * 10;
-    const int y = y0 - 1 + hy, x = x0 - 1 + hx;
-    vin[k] = v < 800 && y >= 0 && y < h && x >= 0 && x < w;  // SAME padding: zeros outside the image
-    voff[k] = vin[k] ? ((size_t)(b * h + y) * w + x) * in_stride + c8 : 0;
-  }
-  auto fetch = [&](int chunk) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      if (vin[k]) {
-        vh[k] = *reinterpret_cast<const uint4*>(in_hi + voff[k] + chunk * 64);
-        vl[k] = *reinterpret_cast<const uint4*>(in_lo + voff[k] + chunk * 64);
-      } else {
-        vh[k] = make_uint4(0, 0, 0, 0);
-        vl[k] = make_uint4(0, 0, 0, 0);
-      }
-    }
-  };
-  fetch(0);
-  for (int chunk = 0; chunk < CIN / 64; ++chunk) {
-    __syncthreads();  // the previous chunk has been consumed (first pass: the weights are in place)
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int v = tid + k * 256;
-      if (v < 800) {
-        const int hp = v >> 3, c8 = (v & 7) * 8;
-        const __half* hh = reinterpret_cast<const __half*>(&vh[k]);
-        const __half* ll = reinterpret_cast<const __half*>(&vl[k]);
-        float f[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) f[i] = join_f32(hh[i], ll[i]);
-        float4* dst = reinterpret_cast<float4*>(&act[hp * kPitch + c8]);
-        dst[0] = make_float4(f[0], f[1], f[2], f[3]);
-        dst[1] = make_float4(f[4], f[5], f[6], f[7]);
-      }
-    }
-    __syncthreads();
-    if (chunk + 1 < CIN / 64) fetch(chunk + 1);
-#pragma unroll
-    for (int t = 0; t < 9; ++t) {
-      const int ky = t / 3, kx = t - ky * 3;
-      const float4* a = reinterpret_cast<const float4*>(&act[((ly + ky) * 10 + lx + kx) * kPitch + q * 16]);
-      const float2* ww = &wsm[t * CIN + chunk * 64 + q * 16];
-#pragma unroll
-      for (int c4 = 0; c4 < 4; ++c4) {
-        const float4 av = a[c4];
-        const float2 u0 = ww[c4 * 4 + 0], u1 = ww[c4 * 4 + 1], u2 = ww[c4 * 4 + 2], u3 = ww[c4 * 4 + 3];
-        acc0 = fmaf(av.x, u0.x, acc0); acc1 = fmaf(av.x, u0.y, acc1);
-        acc0 = fmaf(av.y, u1.x, acc0); acc1 = fmaf(av.y, u1.y, acc1);
-        acc0 = fmaf(av.z, u2.x, acc0); acc1 = fmaf(av.z, u2.y, acc1);
-        acc0 = fmaf(av.w, u3.x, acc0); acc1 = fmaf(av.w, u3.y, acc1);
-      }
-    }
-  }
-  if (trigger == 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  red[q][px] = make_float2(acc0, acc1);
-  __syncthreads();
-  if (tid < 64) {
-    const int y = y0 + ly, x = x0 + lx;
-    if (y < h && x < w) {
-      const float2 r0 = red[0][px], r1 = red[1][px], r2 = red[2][px], r3 = red[3][px];
-      const float d0 = ((r0.x + r1.x) + (r2.x + r3.x)) + bias[0];
-      const float d1 = ((r0.y + r1.y) + (r2.y + r3.y)) + bias[1];
-      const size_t o = ((size_t)(b * h + y) * w + x) * 2;
-      float2 c = *reinterpret_cast<float2*>(coords1 + o);
-      c.x += d0; c.y += d1;
-      *reinterpret_cast<float2*>(coords1 + o) = c;
-      if (delta_out) *reinterpret_cast<float2*>(delta_out + o) = make_float2(d0, d1);
-    }
-  }
-}
-
-static int launch_flow_head2(const ConvParams& p, cudaStream_t s) {
-  static const int pdl = getenv("RAFT_B200_NO_PDL") ? 0 : 1;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((p.w + 7) / 8, (p.h + 7) / 8, p.B);
-  cfg.blockDim = dim3(256);
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl;
-  // when the dependents (next iteration's lookup / convc1) may be scheduled: 0 = kernel start, 1 = after the FMA loop,
-  // 2 = at completion (tuning knob)
-  static const int trigger = getenv("RAFT_B200_FH2_TRIGGER") ? atoi(getenv("RAFT_B200_FH2_TRIGGER")) : 1;
-  if (p.cin_pad == 256) {
-    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, flow_head2_kernel<256>, p.in_hi, p.in_lo, p.in_stride, p.w_hi, p.w_lo, p.bias, p.f1,
-                                     p.f2, p.h, p.w, trigger));
-  } else {
-    RB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, flow_head2_kernel<128>, p.in_hi, p.in_lo, p.in_stride, p.w_hi, p.w_lo, p.bias, p.f1,
-                                     p.f2, p.h, p.w, trigger));
-  }
-  RB_CHECK_LAUNCH("flow_head2_kernel");
-  return RB_OK;
-}
-
 // Phase-timestamp debug buffer (tools/phase_times.py): rb_debug_set_buffer(ptr, convs) makes the next update
 // step record 8 timestamps per CTA for each of its convs, in launch order, 4096 CTAs per conv.
 static thread_local long long* g_dbg = nullptr;
 static thread_local int g_dbg_idx = 0;
-#ifdef RB_EXPERIMENTS
-// Fused mode (experiment build only, RAFT_B200_FUSED=1): the convs of one update step are recorded into a job list and
-// run as ONE persistent kernel with grid barriers between dependent convs (experiments/update_fused.cu).
-static thread_local FusedJobs* g_rec = nullptr;
-static thread_local int g_rec_wait = 1, g_rec_offset = 0;
-static inline bool fused_mode() {
-  static const bool on = getenv("RAFT_B200_FUSED") != nullptr;
-  return on && math_mode() == RB_MATH_TC;
-}
-#else
-static inline constexpr bool fused_mode() { return false; }
-#endif
 static int launch_conv_dbg(ConvParams& p, cudaStream_t s) {
-  static const int early = getenv("RAFT_B200_PDL_EARLY") ? 1 : 0;
-#ifdef RB_EXPERIMENTS
-  if (g_rec) {
-    RB_REQUIRE(g_rec->n < kMaxFusedJobs, RB_ERR_UNSUPPORTED, "fused update: too many convs");
-    FusedJob& jb = g_rec->job[g_rec->n];
-    p.whatif = g_rec->whatif;
-    int rc = conv_tc_prepare(p, &jb);
-    if (rc) return rc;
-    jb.wait_prev = g_rec_wait;
-    jb.cta_offset = g_rec_offset;
-    g_rec->n++;
-    return RB_OK;
-  }
-#endif
-  p.pdl_early = early;
   if (g_dbg) p.dbg = g_dbg + (size_t)(g_dbg_idx++) * 4096 * 8;
   return launch_conv(p, s);
 }
@@ -574,36 +406,21 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
   const int foff = xoff + v.mo_out;       // channel offset of the raw flow
   int rc;
   g_dbg_idx = 0;
-  const bool fused = fused_mode();
-#ifdef RB_EXPERIMENTS
-  FusedJobs jobs;
-  if (fused) {
-    static const int whatif = getenv("RAFT_B200_WHATIF") ? atoi(getenv("RAFT_B200_WHATIF")) : 0;
-    jobs.n = 0; jobs.counters = W.counters; jobs.whatif = whatif; jobs.dbg = g_dbg;
-    static const int st = getenv("RAFT_B200_FUSED_STAGES") ? atoi(getenv("RAFT_B200_FUSED_STAGES")) : 3;
-    jobs.stages = st < 1 ? 1 : (st > 3 ? 3 : st); g_rec_wait = 1; g_rec_offset = 0;
-  }
-  struct RecGuard {  // recording never outlives this call, whatever the exit path
-    ~RecGuard() { g_rec = nullptr; }
-  } rec_guard;
-#endif
   // ---- motion encoder (model_utils.py:110-129) ----
   SideStream* ss;
   if ((rc = side_stream(&ss))) return rc;
   RB_CHECK_CUDA(cudaEventRecord(ss->fork, s));
   RB_CHECK_CUDA(cudaStreamWaitEvent(ss->stream, ss->fork, 0));
   {  // flow branch (side stream): convf1 (7x7) -> convf2
-    static const int seg_env = getenv("RAFT_B200_CONV7_SEG") ? atoi(getenv("RAFT_B200_CONV7_SEG")) : 0;  // tuning knob
-    const int seg = seg_env ? seg_env : ((long)B * h * w <= 16384 ? 16 : 32);  // same-box A/B at 55x128: 792 / 772 / 781 us per 4 iterations for 32 / 16 / 8
+    const int seg = (long)B * h * w <= 16384 ? 16 : 32;  // same-box A/B at 55x128: 792 / 772 / 781 us per 4 iterations for 32 / 16 / 8
     const float* Wf = reinterpret_cast<const float*>(bb + L.f1_w);
     const float* bf = reinterpret_cast<const float*>(bb + L.f1_b);
     const float2* c1 = reinterpret_cast<const float2*>(coords1);
 #define RB_LAUNCH_CONV7(COUT, SEG) \
     flow_conv7_kernel<COUT, SEG><<<dim3((w + SEG - 1) / SEG, h, B), COUT, 0, ss->stream>>>(c1, Wf, bf, W.f1, v.f1, W.hx, W.qx, v.hx, foff, h, w)
-    // default: convf1 on the tensor cores (flow_prep_kernel + 7x1 conv over the window view); RAFT_B200_CONVF1_SIMT=1, the
-    // CUDA-core math mode and the fused experiment keep the CUDA-core kernel
-    static const bool f1_simt = getenv("RAFT_B200_CONVF1_SIMT") != nullptr;
-    const bool f1_tc = !f1_simt && !fused && math_mode() == RB_MATH_TC && (foff & 1) == 0 && (v.hx & 1) == 0 && w >= 8;
+    // convf1 on the tensor cores (flow_prep_kernel + 7x1 conv over the window view); the CUDA-core math mode and grids
+    // narrower than the window keep the CUDA-core kernel
+    const bool f1_tc = math_mode() == RB_MATH_TC && (foff & 1) == 0 && (v.hx & 1) == 0 && w >= 8;
     if (f1_tc) {
       const size_t cells = (size_t)B * h * (w + 8);
       flow_prep_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, ss->stream>>>(c1, W.fl, W.hx, W.qx, v.hx, foff, B, h, w);
@@ -620,25 +437,23 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
       p.cout = L.f1t_cout; p.cout_pad = L.f1t_cout_pad;
       p.B = B; p.h = h; p.w = w; p.hidden = v.hidden; p.scale = 1.f;
       set_act(p, ACT_RELU, W.f1, v.f1, 0);
-      static const int lim1 = getenv("RAFT_B200_CONVF1_CTAS") ? atoi(getenv("RAFT_B200_CONVF1_CTAS")) : -1;  // tuning knob
       // batch 1: 28 CTAs = the 55 128-wide tiles in two full rounds (same-box sweep of both budgets, 4 iterations:
       // 19/38: 650, 28/28: 633, 28/38: 632, 38/38: 637, 55/38: 651, 38/55: 650, 110/38: 649 us)
-      p.cta_limit = lim1 >= 0 ? lim1 : ((long)B * h * w <= 16384 ? 28 : 0);
+      p.cta_limit = (long)B * h * w <= 16384 ? 28 : 0;
       if ((rc = launch_conv_dbg(p, ss->stream))) return rc;
     } else if (v.small) {
-      if (seg == 8) RB_LAUNCH_CONV7(64, 8); else if (seg == 16) RB_LAUNCH_CONV7(64, 16); else RB_LAUNCH_CONV7(64, 32);
+      if (seg == 16) RB_LAUNCH_CONV7(64, 16); else RB_LAUNCH_CONV7(64, 32);
     } else {
-      if (seg == 8) RB_LAUNCH_CONV7(128, 8); else if (seg == 16) RB_LAUNCH_CONV7(128, 16); else RB_LAUNCH_CONV7(128, 32);
+      if (seg == 16) RB_LAUNCH_CONV7(128, 16); else RB_LAUNCH_CONV7(128, 32);
     }
 #undef RB_LAUNCH_CONV7
     RB_CHECK_LAUNCH("flow_conv7_kernel");
-    if (!fused) {
+    {
       ConvParams p = base_params(v, L, blob, P_CONVF2, W.f1, v.f1, 0, B, h, w);
       set_act(p, ACT_RELU, W.cf, v.cf, v.cor);
       // convf2 runs beside convc1 / convc2 of the main stream: a small CTA budget keeps it off the SMs they need
       // (batch 1: the other convs use 110 of the 148 SMs; same-box A/B 770 -> 761 us per 4 iterations)
-      static const int lim = getenv("RAFT_B200_CONVF2_CTAS") ? atoi(getenv("RAFT_B200_CONVF2_CTAS")) : -1;  // tuning knob
-      p.cta_limit = lim >= 0 ? lim : ((long)B * h * w <= 16384 ? 38 : 0);
+      p.cta_limit = (long)B * h * w <= 16384 ? 38 : 0;
       if ((rc = launch_conv_dbg(p, ss->stream))) return rc;
     }
     RB_CHECK_CUDA(cudaEventRecord(ss->join, ss->stream));
@@ -647,33 +462,10 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
   if (pyramid) {
     if ((rc = launch_lookup(pyramid, coords1, nullptr, W.corr.hi, W.corr.lo, v.corr_pad, B, h, w, v.radius, s))) return rc;
   }
-#ifdef RB_EXPERIMENTS
-  if (fused) {
-    // both branches (flow_conv7 on the side stream, the lookup here) end before the fused kernel starts; its first two
-    // jobs (convc1, convf2) are independent of each other and are spread over different CTAs
-    RB_CHECK_CUDA(cudaStreamWaitEvent(s, ss->join, 0));
-    g_rec = &jobs;
-    g_rec_wait = 0;
-  }
-  auto record_convf2 = [&]() -> int {
-    if (!fused) return RB_OK;
-    ConvParams p = base_params(v, L, blob, P_CONVF2, W.f1, v.f1, 0, B, h, w);
-    set_act(p, ACT_RELU, W.cf, v.cf, v.cor);
-    g_rec_offset = jobs.job[0].g.total_tiles;
-    int r = launch_conv_dbg(p, s);
-    g_rec_offset = 0;
-    g_rec_wait = 1;
-    return r;
-  };
-#else
-  auto record_convf2 = []() -> int { return RB_OK; };
-#endif
   if (!v.small) {
     ConvParams p = base_params(v, L, blob, P_CONVC1, W.corr, v.corr_pad, 0, B, h, w);
     set_act(p, ACT_RELU, W.c1, v.c1, 0);
     if ((rc = launch_conv_dbg(p, s))) return rc;
-    rc = record_convf2();
-    if (rc) return rc;
     p = base_params(v, L, blob, P_CONVC2, W.c1, v.c1, 0, B, h, w);
     set_act(p, ACT_RELU, W.cf, v.cf, 0);
     if ((rc = launch_conv_dbg(p, s))) return rc;
@@ -681,10 +473,8 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
     ConvParams p = base_params(v, L, blob, P_CONVC1, W.corr, v.corr_pad, 0, B, h, w);
     set_act(p, ACT_RELU, W.cf, v.cf, 0);
     if ((rc = launch_conv_dbg(p, s))) return rc;
-    rc = record_convf2();
-    if (rc) return rc;
   }
-  if (!fused) RB_CHECK_CUDA(cudaStreamWaitEvent(s, ss->join, 0));
+  RB_CHECK_CUDA(cudaStreamWaitEvent(s, ss->join, 0));
   {
     ConvParams p = base_params(v, L, blob, P_MOTION, W.cf, v.cf, 0, B, h, w);
     set_act(p, ACT_RELU, W.hx, v.hx, xoff);
@@ -728,15 +518,7 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
     // otherwise, so batched and per-sample runs stay bit-identical).  RAFT_B200_NO_SPLITK=1: one accumulator.
     static const bool no_splitk = getenv("RAFT_B200_NO_SPLITK") != nullptr;
     p.split_k = no_splitk ? 0 : 1;
-    // RAFT_B200_FH2_SIMT=1: CUDA-core kernel instead of the N=16 implicit GEMM (profiles/r01_notes.md) -> opt-in.
-    static const bool fh2_simt = getenv("RAFT_B200_FH2_SIMT") != nullptr;
-    const bool direct = !fused && fh2_simt && p.kh == 3 && p.kw == 3 && p.in_choff == 0 && p.in_stride % 8 == 0 &&
-                        (p.cin_pad == 256 || p.cin_pad == 128) && p.cout == 2;
-    if (direct) {
-      if ((rc = launch_flow_head2(p, s))) return rc;
-    } else if ((rc = launch_conv_dbg(p, s))) {
-      return rc;
-    }
+    if ((rc = launch_conv_dbg(p, s))) return rc;
   }
   // ---- mask head (model_utils.py:180-183); only the last iteration's mask is ever consumed ----
   if (mask_out) {
@@ -748,12 +530,6 @@ static int update_step(const Variant& v, const void* blob, void* wsp, float* coo
     p.epi = EPI_F32; p.f0 = mask_out; p.scale = 0.25f;
     if ((rc = launch_conv_dbg(p, s))) return rc;
   }
-#ifdef RB_EXPERIMENTS
-  if (fused) {
-    g_rec = nullptr;
-    if ((rc = launch_fused_jobs(jobs, s))) return rc;
-  }
-#endif
   return RB_OK;
 }
 

@@ -1,11 +1,7 @@
-"""Feature / context encoders (networks/model_utils.py:6-105) on stock torch/cuDNN ops.
+"""Feature / context encoders (networks/model_utils.py:6-105) on raft_b200's own kernels (csrc/encoder.cu).
 
-SURVEY section 2 row 8 / section 8(f) F1: the encoders run once per pair and are NOT part of the
-hand-written hot path this round; they are required for an end-to-end flow, so they are restated
-with exact TF semantics (asymmetric 'SAME' padding on the stride-2 convs, instance norm without
-affine, BatchNorm with EMA statistics) in fp32 with TF32 disabled.  Tensors are NCHW
-(channels_last memory format) internally; the public functions take and return NHWC like the
-reference.
+Exact TF semantics: asymmetric 'SAME' padding on the stride-2 convs, instance norm without affine, BatchNorm with EMA
+statistics.  Frames go in and feature maps come out NHWC, like the reference.
 """
 from __future__ import annotations
 
@@ -13,79 +9,12 @@ from typing import Dict
 
 import numpy as np
 import torch
-import torch.nn.functional as F
-
-
-def _same_pad(n: int, k: int, s: int):
-    out = -(-n // s)
-    total = max((out - 1) * s + k - n, 0)
-    return total // 2, total - total // 2
-
-
-class Encoder:
-    """BasicEncoder (things) / SmallEncoder (small) with weights keyed like the reference npz."""
-
-    def __init__(self, params: Dict[str, np.ndarray], name: str, small: bool, norm_fn: str, device):
-        self.name, self.small, self.norm_fn = name, small, norm_fn
-        self.p = {}
-        for k, v in params.items():
-            if not k.startswith(name + "/"):
-                continue
-            t = torch.as_tensor(np.asarray(v, dtype=np.float32), device=device)
-            if k.endswith("/W"):
-                t = t.permute(3, 2, 0, 1).contiguous(memory_format=torch.channels_last)  # HWIO -> OIHW
-            self.p[k] = t
-
-    def _conv(self, x, scope, stride=1):
-        W, b = self.p[scope + "/W"], self.p[scope + "/b"]
-        kh, kw = W.shape[2], W.shape[3]
-        pt, pb = _same_pad(x.shape[2], kh, stride)
-        pl, pr = _same_pad(x.shape[3], kw, stride)
-        if pt == pb and pl == pr:
-            return F.conv2d(x, W, b, stride=stride, padding=(pt, pl))
-        return F.conv2d(F.pad(x, (pl, pr, pt, pb)), W, b, stride=stride)
-
-    def _norm(self, x, scope):
-        if self.norm_fn == "instance":
-            return F.instance_norm(x, eps=1e-5)
-        if self.norm_fn == "batch":
-            p = self.p
-            return F.batch_norm(x, p[scope + "/mean/EMA"], p[scope + "/variance/EMA"], p[scope + "/gamma"],
-                                p[scope + "/beta"], training=False, eps=1e-5)
-        return x
-
-    def _residual(self, x, scope, stride):  # model_utils.py:19-35
-        y = torch.relu(self._norm(self._conv(x, scope + "/conv1", stride), scope + "/norm1"))
-        y = torch.relu(self._norm(self._conv(y, scope + "/conv2", 1), scope + "/norm2"))
-        if stride != 1:
-            x = self._norm(self._conv(x, scope + "/downsample.0", stride), scope + "/downsample.1")
-        return torch.relu(x + y)
-
-    def _bottleneck(self, x, scope, stride):  # model_utils.py:37-57
-        y = torch.relu(self._norm(self._conv(x, scope + "/conv1", 1), scope + "/norm1"))
-        y = torch.relu(self._norm(self._conv(y, scope + "/conv2", stride), scope + "/norm2"))
-        y = torch.relu(self._norm(self._conv(y, scope + "/conv3", 1), scope + "/norm3"))
-        if stride != 1:
-            x = self._norm(self._conv(x, scope + "/downsample.0", stride), scope + "/downsample.1")
-        return torch.relu(x + y)
-
-    def __call__(self, img_nhwc: torch.Tensor) -> torch.Tensor:
-        """[B,H,W,3] in [-1,1] -> [B,H/8,W/8,C] NHWC contiguous fp32."""
-        n = self.name
-        x = img_nhwc.permute(0, 3, 1, 2)  # NCHW view of NHWC memory == channels_last
-        x = torch.relu(self._norm(self._conv(x, n + "/conv1", 2), n + "/norm1"))
-        block = self._bottleneck if self.small else self._residual
-        for lname, stride in (("layer1", 1), ("layer2", 2), ("layer3", 2)):
-            x = block(x, f"{n}/{lname}/0", stride)
-            x = block(x, f"{n}/{lname}/1", 1)
-        x = self._conv(x, n + "/conv2", 1)
-        return x.permute(0, 2, 3, 1).contiguous()
 
 
 class CudaEncoder:
-    """The same encoders on raft_b200's own kernels (csrc/encoder.cu): every conv runs on the tcgen05
-    implicit-GEMM kernel of the update block (split fp16 operands), instance norm as a fused
-    stats/apply pass, batch norm folded into the weights.  Same call signature as ``Encoder``."""
+    """BasicEncoder (things) / SmallEncoder (small) with weights keyed like the reference npz: every conv runs on the
+    tcgen05 implicit-GEMM kernel of the update block (split fp16 operands), instance norm as a fused stats/apply pass,
+    batch norm folded into the weights."""
 
     NORMS = {"none": 0, "instance": 1, "batch": 2}
 

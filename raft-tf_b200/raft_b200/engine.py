@@ -3,7 +3,6 @@
 rb_encoder_forward x2 (fnet on both frames, cnet on a forked stream; csrc/encoder.cu) -> rb_corr_build ->
 rb_update_set_state_cnet -> rb_raft_iterate (lookup + update block per iteration) -> rb_upsample_convex /
 rb_upflow8, all replayed from ONE CUDA graph.  Mirrors RAFT.network_graph (networks/RAFT.py:78-109).
-The torch/cuDNN restatement of the encoders (encoders.Encoder) is a cross-check behind RAFT_B200_TORCH_ENCODERS=1.
 """
 from __future__ import annotations
 
@@ -14,7 +13,7 @@ import numpy as np
 import torch
 
 from . import capi
-from .encoders import CudaEncoder, Encoder
+from .encoders import CudaEncoder
 from .weights import pack_update_block
 
 
@@ -33,18 +32,10 @@ class RaftEngine:
         # costs ~100 k extra FMA per pixel and iteration on the CUDA cores; same flow up to fp32 summation order.
         self.volume_free = bool(os.environ.get("RAFT_B200_VOLUME_FREE")) if volume_free is None else bool(volume_free)
         self.math_mode = math_mode
-        torch.backends.cudnn.allow_tf32 = False  # the reference is fp32 end to end (only matters for the cuDNN cross-check)
-        torch.backends.cuda.matmul.allow_tf32 = False
-        # encoders: raft_b200's own kernels by default; RAFT_B200_TORCH_ENCODERS=1 selects the torch/cuDNN restatement
-        self.torch_encoders = bool(os.environ.get("RAFT_B200_TORCH_ENCODERS"))
         cnorm = "none" if small else "batch"
         with torch.cuda.device(self.device):
-            if self.torch_encoders:
-                self.fnet = Encoder(params, "fnet", small, "instance", self.device)
-                self.cnet = Encoder(params, "cnet", small, cnorm, self.device)
-            else:
-                self.fnet = CudaEncoder(params, "fnet", small, "instance", self.fdim, self.device)
-                self.cnet = CudaEncoder(params, "cnet", small, cnorm, self.hidden + self.ctx, self.device)
+            self.fnet = CudaEncoder(params, "fnet", small, "instance", self.fdim, self.device)
+            self.cnet = CudaEncoder(params, "cnet", small, cnorm, self.hidden + self.ctx, self.device)
             self.blob = pack_update_block(params, small, self.device)
         self._shape = None
         self._graph = None
@@ -104,25 +95,17 @@ class RaftEngine:
         if self.staged:  # F3: u8 -> fp32 /255 and replicate padding in one pass (csrc/frames.cu)
             capi.check(capi.lib.rb_frames_prepare(capi.ptr(self.raw), int(u8), capi.ptr(self.images), 2 * B, H, W,
                                                   *self.pad, capi.stream()))
-        if self.torch_encoders:
-            both = self.images * 2.0 - 1.0
-            self.fmaps.copy_(self.fnet(both))  # instance norm is per sample, so batching left|right is exact
-            self.cmap.copy_(self.cnet(both[:B]))
-        elif os.environ.get("RAFT_B200_SERIAL_ENCODERS"):
-            self.fnet(self.images, out=self.fmaps)
+        main = torch.cuda.current_stream(self.device)
+        if self._enc_stream is None:
+            self._enc_stream = torch.cuda.Stream(device=self.device)
+        side = self._enc_stream
+        side.wait_stream(main)  # fork: the frames are in place
+        with torch.cuda.stream(side):
             self.cnet(self.images[:B], out=self.cmap)
-        else:
-            main = torch.cuda.current_stream(self.device)
-            if self._enc_stream is None:
-                self._enc_stream = torch.cuda.Stream(device=self.device)
-            side = self._enc_stream
-            side.wait_stream(main)  # fork: the frames are in place
-            with torch.cuda.stream(side):
-                self.cnet(self.images[:B], out=self.cmap)
-            self.fnet(self.images, out=self.fmaps)
-            self._cnet_pending = True
-            if not defer_join:
-                self._join_cnet()
+        self.fnet(self.images, out=self.fmaps)
+        self._cnet_pending = True
+        if not defer_join:
+            self._join_cnet()
 
     def _join_cnet(self):
         if self._cnet_pending:
@@ -164,8 +147,7 @@ class RaftEngine:
         self._hot_path()
 
     def launches_per_forward(self) -> int:
-        """Number of raft_b200 kernels one forward pass launches (counted by the library; torch kernels of
-        the optional cuDNN encoder path are not included)."""
+        """Number of raft_b200 kernels one forward pass launches (counted by the library)."""
         capi.lib.rb_launch_count_reset()
         with torch.cuda.device(self.device):
             self._all()
@@ -173,17 +155,12 @@ class RaftEngine:
         return int(capi.lib.rb_launch_count())
 
     def run(self):
-        """encoders + hot path on self.images; replayed from one CUDA graph when every stage is ours."""
+        """encoders + hot path on self.images, replayed from one CUDA graph."""
         if not self.use_graph:
             self._all()
             return
-        if self.torch_encoders:  # cuDNN autotuning does not belong in a capture: graph only the hot path
-            self.encode()
-            body = self._hot_path
-        else:
-            body = self._all
         if self._graph is None:
-            body()  # warm-up: function attributes, tensor-map cache
+            self._all()  # warm-up: function attributes, tensor-map cache
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             # torch.cuda.graph's default capture stream is a process-wide singleton on whichever device used it first, and
@@ -192,7 +169,7 @@ class RaftEngine:
             if self._capture_stream is None:
                 self._capture_stream = torch.cuda.Stream(device=self.device)
             with torch.cuda.graph(g, stream=self._capture_stream):
-                body()
+                self._all()
             self._graph = g
         self._graph.replay()
 

@@ -22,6 +22,14 @@ def test_library_exports_every_declared_symbol():
     assert set(names) == set(capi.SIGNATURES), set(names) ^ set(capi.SIGNATURES)
 
 
+def test_library_reads_only_the_documented_knobs():
+    """The environment variables the library reads: the switches README.md lists, nothing left over from tuning."""
+    from raft_b200 import capi
+    names = set(re.findall(rb"RAFT_B200_[A-Z0-9_]+", open(capi.LIB_PATH, "rb").read()))
+    assert names == {b"RAFT_B200_" + k for k in (b"NO_PDL", b"NO_HOIST", b"NO_STASH", b"NO_SPLITK", b"NO_SPLITK_CLUSTER",
+                                                   b"NO_FUSED_STATS", b"LOOKUP_V5", b"SPLITK_CLOSING_BARRIER")}, names
+
+
 def test_host_only_queries():
     from raft_b200 import capi
     lib = capi.lib

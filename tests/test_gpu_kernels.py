@@ -252,13 +252,15 @@ def test_conv2d_stride2(cuda, mode, case):
                                  capi.stream()) == -3  # RB_ERR_UNSUPPORTED: stride 3
 
 
+# (1, 9, 6): grids narrower than the 8-pixel window of the tensor-core convf1 run flow_conv7_kernel beside the
+# tensor-core convs
+@pytest.mark.parametrize("B,h,w", [(2, 12, 20), (1, 9, 6)])
 @pytest.mark.parametrize("mode", ["tc", "simt"])
 @pytest.mark.parametrize("small", [False, True])
-def test_update_block(cuda, mode, small):
+def test_update_block(cuda, mode, small, B, h, w):
     """BasicUpdateBlock / SmallUpdateBlock (model_utils.py:172-194): (net, mask, delta_flow)."""
     from raft_b200 import capi, synth
     from networks import model_utils as MU
-    B, h, w = 2, 12, 20
     hid, ctx, r = (96, 64, 3) if small else (128, 128, 4)
     K = 4 * (2 * r + 1) ** 2
     p = synth.make_weights(small)
