@@ -187,6 +187,16 @@ int rb_upflow8_crop(const float* coords1, float* out, int B, int h, int w, float
 int rb_frames_prepare(const void* src, int src_is_u8, float* dst, int B, int H, int W, int pad_top,
                       int pad_bottom, int pad_left, int pad_right, void* stream);
 
+/* ---- F5 (output edge): forward-backward consistency (occlusion) check, both directions in one launch -----------
+ * flow_fw, flow_bw: [B,H,W,2] fp32 (x, y), 8-byte aligned; occ_fw, occ_bw: [B,H,W] uint8.  Displacements are scale*flow
+ * pixels (8.0 for raft-small's flow, which keeps the reference's missing x8 of upflow8, utils.py:105-111; 1.0 for
+ * raft-things).  For each direction with flow f and the other direction's flow g, at pixel p: u = scale*f(p), t = p + u;
+ * occ = 2 if t lies outside [0,W-1] x [0,H-1]; else g' = scale*bilinear(g, t) (corners floor(t) and min(floor(t)+1, dim-1))
+ * and occ = 1 if |u + g'|^2 >= alpha1 (|u|^2 + |g'|^2) + alpha2, otherwise 0 (Sundaram et al. 2010, UnFlow).
+ * scale > 0, alpha1 >= 0, alpha2 >= 0. */
+int rb_flow_consistency(const float* flow_fw, const float* flow_bw, uint8_t* occ_fw, uint8_t* occ_bw, int B, int H,
+                        int W, float scale, float alpha1, float alpha2, void* stream);
+
 /* ---- F1: BasicEncoder / SmallEncoder  networks/model_utils.py:61-105 (+ input_preprocess RAFT.py:53-59) --
  * norm: 0 = 'none', 1 = 'instance' (fnet), 2 = 'batch' (cnet of raft-things; folded into the convs at pack
  * time from inference statistics).  Convs are enumerated in execution order; names are relative to the

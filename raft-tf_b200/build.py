@@ -7,7 +7,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = ["capi.cu", "corr.cu", "conv_simt.cu", "conv_tc.cu", "conv_api.cu", "gemm_tc.cu", "update.cu", "upsample.cu",
-           "encoder.cu", "frames.cu"]
+           "encoder.cu", "frames.cu", "consistency.cu"]
 LIB = os.path.join(HERE, "lib", "libraft_b200.so")
 
 

@@ -90,8 +90,24 @@ class RAFT(object):
         uint8 in [0,255] (extension: the /255 of test_dataflow.py:96-97 then runs on the GPU); numpy or torch, host or
         CUDA -> [B,H,W,2] torch CUDA flow (a fresh tensor per call, like a session.run result).  H, W that are not
         multiples of 8 are replicate-padded and the flow cropped back, both inside the engine's own kernels."""
-        def as_tensor(x):
-            t = torch.as_tensor(x)
-            return t if t.dtype == torch.uint8 else t.to(torch.float32)
-        flow = self.engine().forward(as_tensor(input_left), as_tensor(input_right))
+        flow = self.engine().forward(_as_frames(input_left), _as_frames(input_right))
         return flow.clone()
+
+    @torch.no_grad()
+    def forward_backward(self, input_left, input_right, alpha1=0.01, alpha2=0.5):
+        """Extension: the flow in both directions and the forward-backward consistency masks, from one CUDA graph that
+        runs the two directions as one batch (the feature maps of each frame are computed once).  Frames as for
+        ``forward``.  Returns fresh CUDA tensors ``(flow_fw, flow_bw, occ_fw, occ_bw)``: flow_fw == forward(left, right)
+        and flow_bw == forward(right, left) bit for bit, [B,H,W,2]; occ_* [B,H,W] uint8 with 0 = consistent,
+        1 = occluded (|u + g|^2 >= alpha1 (|u|^2 + |g|^2) + alpha2, u the displacement at p and g the other direction's
+        flow sampled bilinearly at p + u, Sundaram et al. 2010 / UnFlow), 2 = p + u leaves the frame.  Displacements are
+        in full-resolution pixels: raft-small's flow, which keeps the reference's missing x8 of upflow8, is scaled by 8
+        for the check only."""
+        flow, occ = self.engine().forward_backward(_as_frames(input_left), _as_frames(input_right), alpha1, alpha2)
+        B = flow.shape[0] // 2
+        return flow[:B].clone(), flow[B:].clone(), occ[:B].clone(), occ[B:].clone()
+
+
+def _as_frames(x):
+    t = torch.as_tensor(x)
+    return t if t.dtype == torch.uint8 else t.to(torch.float32)

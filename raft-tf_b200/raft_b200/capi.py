@@ -62,6 +62,7 @@ SIGNATURES = {
     "rb_upsample_convex_crop": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "rb_upflow8_crop": (_i, [_vp, _vp, _i, _i, _i, _f, _i, _i, _i, _i, _vp]),
     "rb_frames_prepare": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "rb_flow_consistency": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "rb_encoder_num_convs": (_i, [_i]),
     "rb_encoder_conv_name": (C.c_char_p, [_i, _i]),
     "rb_encoder_norm_name": (C.c_char_p, [_i, _i]),
